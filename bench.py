@@ -21,14 +21,20 @@ BASELINE.json metric: "frames/sec (extract+match+pose-LM) 640x480".  Configurati
   extra_configs  (default run only) a short run of the kitti and euroc configurations on the same GPUs
 
 `--impl reference` times the CPU oracle of the same path on the host threads this process may use.
+`--steps K` is the number of timed steps of every timed loop (the headline, e2e and extra_configs).
+`--dump-outputs DIR` writes what the last timed step of the headline configuration computed to DIR/<name>.npy (see dump_outputs).
+Nothing is written inside the tree: the -march=native oracle of the CPU legs is built in a temporary directory.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
+
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -90,12 +96,19 @@ def make_inputs(B, seed, w=W, h=H, K=None):
 
 
 # ------------------------------------------------------------------------------------------------ CPU oracle arm
+_NATIVE_DIR = None
+
+
 def use_native_oracle():
     """The CPU legs time the -march=native build of the oracle (BASELINE.md §3: -O3 -march=native), compiled on the box that
     does the timing; the portable build that travels with the repo stays the checker of the tests."""
-    lib = os.path.join(ROOT, "oracle", "liboracle_native.so")
+    global _NATIVE_DIR
+    if _NATIVE_DIR is None:
+        _NATIVE_DIR = tempfile.TemporaryDirectory(prefix="plslam-bench-")
+    lib = os.path.join(_NATIVE_DIR.name, "liboracle_native.so")
     try:
-        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "native", f"NATIVE_LIB={lib}"],
+                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         os.environ["PLSLAM_ORACLE_LIB"] = lib
         return "-O3 -march=native"
     except Exception:
@@ -307,7 +320,46 @@ class Ctx:
             self.dist.barrier()
 
 
-def run_config(ctx, name, steps, warmup, batch=None, full=True):
+DUMP_FRAMES = 64           # frames of the batch whose per-feature outputs --dump-outputs writes (fixed seed, sorted)
+
+
+def dump_outputs(fe, B, out_dir):
+    """What the last timed step computed, as a caller of the device-resident path fetches it (Frontend.fetch and fetch_tracking),
+    written as out_dir/<name>.npy in float32 / float64.  Per-frame counts and poses cover the whole batch; per-feature arrays
+    (keypoints, descriptors, keylines, matches) cover DUMP_FRAMES frames drawn with a fixed seed, with the entries past each
+    frame's count zeroed (they are unused buffer space).  Integers are stored as float64, exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    o = fe.fetch(B)
+    t = [fe.fetch_tracking(B, which) for which in (0, 1)]
+    frames = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_FRAMES), replace=False))
+
+    def valid(a, n):              # a[frames] with entries at or past the frame's count zeroed
+        a = a[frames].copy()
+        a[np.arange(a.shape[1])[None, :] >= n[frames][:, None]] = 0
+        return a
+
+    def fields(a):                # structured records -> [..., n_fields]
+        return np.stack([a[f].astype(np.float64) for f in a.dtype.names], -1)
+
+    arrays = {"frames": frames, "n_keypoints": o["n"], "n_keylines": o["nl"], "n_point_matches": o["n_pt_matches"],
+              "n_line_matches": o["n_line_matches"], "poses": o["poses"], "inliers": o["inliers"],
+              "keypoints": fields(valid(o["kps"], o["n"])), "descriptors": valid(o["desc"], o["n"]),
+              "keylines": fields(valid(o["keylines"], o["nl"])), "line_descriptors": valid(o["ldesc"], o["nl"]),
+              "point_matches": valid(o["pt_matches"], o["n"]), "line_matches": valid(o["line_matches"], o["nl"])}
+    for k, tk in enumerate(t):
+        arrays[f"tracking{k}_n_point"] = tk["n_pt"]
+        arrays[f"tracking{k}_n_line"] = tk["n_line"]
+        arrays[f"tracking{k}_point_match"] = valid(tk["pt_match"], o["n"])
+        arrays[f"tracking{k}_line_match"] = valid(tk["line_match"], o["nl"])
+    total = 0
+    for k, a in arrays.items():
+        a = np.ascontiguousarray(a, np.float32 if a.dtype in (np.float32, np.uint8) else np.float64)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    assert total <= 64 << 20, total
+
+
+def run_config(ctx, name, steps, warmup, batch=None, full=True, dump_dir=None):
     """One configuration on this process's GPU; returns the measurements (rank-local python values, timings max over ranks)."""
     import plslam_b200 as pl
     from plslam_b200 import synth, sharding
@@ -371,6 +423,8 @@ def run_config(ctx, name, steps, warmup, batch=None, full=True):
     ms = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     launches = pl.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(fe, B, dump_dir)
     res = dict(name=name, B=B, total=total, halo=halo, ms=ms, steps=steps, value=total * steps / (ms / 1000.0), launches=int(launches),
                clocks=clocks, frame=[w, h], orb=list(cfg["orb"]))
     if ba is not None:
@@ -406,7 +460,7 @@ def run_config(ctx, name, steps, warmup, batch=None, full=True):
     fe.wait(0)
     torch.cuda.synchronize()
     ctx.barrier()
-    e2e_steps = max(3, min(steps, 6))
+    e2e_steps = steps
     t0 = time.perf_counter()
     for k in range(e2e_steps):
         fe.upload_pose_problems(None)      # the step's LM problems travel with the step (14 KB per frame)
@@ -469,7 +523,7 @@ def cpu_baseline_single_thread(frames, problems):
 def run_ours(args):
     ctx = Ctx()
     name = args.config
-    res = run_config(ctx, name, args.steps, args.warmup, args.batch, full=True)
+    res = run_config(ctx, name, args.steps, args.warmup, args.batch, full=True, dump_dir=args.dump_outputs)
     cfg = CONFIGS[name]
     latency, extra, cpu = None, None, None
     if ctx.world == 1 and name == "tum":
@@ -477,7 +531,7 @@ def run_ours(args):
     if name == "tum" and not args.no_extra:
         extra = {}
         for other in ("kitti", "euroc"):
-            r = run_config(ctx, other, 3, 3, None, full=False)
+            r = run_config(ctx, other, args.steps, 3, None, full=False)
             extra[other] = {"value": r["value"], "unit": "frames/s", "ms_per_step": r["ms"] / r["steps"], "frames_per_step_total": r["total"],
                             "frames_this_rank": r["B"], "halo": r["halo"], "scaling": "strong", "frame": r["frame"], "orb": r["orb"],
                             **({"lba_ms": r["lba_ms"], "lba_window": r["lba_window"]} if "lba_ms" in r else {})}
@@ -557,6 +611,8 @@ def main():
     ap.add_argument("--config", default="tum", choices=sorted(CONFIGS), help="BASELINE.json configuration (tum = the headline metric)")
     ap.add_argument("--no-extra", action="store_true", help="default run: skip the short kitti / euroc runs")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

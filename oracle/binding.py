@@ -4,6 +4,8 @@ import os
 import subprocess
 import numpy as np
 
+from . import recorded as _rec
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "liboracle.so")
 
@@ -75,6 +77,7 @@ def ref_line_lib():
     return _ref_line
 
 
+@_rec.entry("ref_lsd_keylines", ref_line_available, ref_only=True)
 def ref_lsd_keylines(img, mask=None, scale=1, num_octaves=1):
     """LSDDetectorC::detect(image, keylines, scale, numOctaves, mask) of the reference tree itself -> KeyLine records
     in detection order (LINEextractor passes scale = (int)1.2 = 1 and one octave)."""
@@ -87,6 +90,7 @@ def ref_lsd_keylines(img, mask=None, scale=1, num_octaves=1):
     return kl[:n].copy()
 
 
+@_rec.entry("ref_line_extract", ref_line_available, ref_only=True)
 def ref_line_extract(img, mask=None, nfeatures=200, min_line_length=0.0):
     """LINEextractor::operator() of the reference itself (src/LineExtractor.cpp) -> (keylines, descriptors, line functions).
     Only for frames with more lines than nfeatures (see oracle/ref_line_wrap.cpp)."""
@@ -101,6 +105,7 @@ def ref_line_extract(img, mask=None, nfeatures=200, min_line_length=0.0):
     return kl[:n].copy(), desc[:n].copy(), lf[:n].copy()
 
 
+@_rec.entry("ref_lbd_compute", ref_line_available, ref_only=True)
 def ref_lbd_compute(img, keylines, want_float=False):
     """BinaryDescriptor::compute(image, keylines, descriptors) of the reference tree itself (class_id must index the lines)."""
     img = np.ascontiguousarray(img, np.uint8); kl = np.ascontiguousarray(keylines)
@@ -132,9 +137,19 @@ def _ref_frame_lib():
     return _ref_frame
 
 
+_frame_key = None      # the arguments of the last ref_frame_construct: ref_frame_features_in_area answers for that frame
+
+
 def ref_frame_construct(img, K, D, mask=None, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20, min_th=7, nlines=200, min_line_length=0.0):
     """The reference's monocular Frame constructor itself (Frame.cc:193-276) -> dict(keys, keysUn, desc, keylines, ldesc, lfunc, bounds,
     grid (start, items), line_grid (start, items)).  The frame stays alive for ref_frame_features_in_area(_line)."""
+    global _frame_key
+    a = (img, K, D, mask, nfeatures, scale_factor, nlevels, ini_th, min_th, nlines, min_line_length)
+    _frame_key = _rec.digest("ref_frame_construct", *a)
+    return _rec.call("ref_frame_construct", a, ref_frame_available(), lambda: _ref_frame_construct(*a))
+
+
+def _ref_frame_construct(img, K, D, mask, nfeatures, scale_factor, nlevels, ini_th, min_th, nlines, min_line_length):
     img = np.ascontiguousarray(img, np.uint8); h, w = img.shape
     cap, capl = 2 * nfeatures + 64, nlines + 2
     counts = np.zeros(2, np.int32)
@@ -158,6 +173,11 @@ def ref_frame_construct(img, K, D, mask=None, nfeatures=1000, scale_factor=1.2, 
 
 
 def ref_frame_features_in_area(x, y, r, min_level=-1, max_level=-1):
+    return _rec.call("ref_frame_features_in_area", (_frame_key, x, y, r, min_level, max_level), ref_frame_available(),
+                     lambda: _ref_frame_features_in_area(x, y, r, min_level, max_level))
+
+
+def _ref_frame_features_in_area(x, y, r, min_level, max_level):
     out = np.zeros(8192, np.int32)
     f = _ref_frame_lib().ref_frame_features_in_area
     f.argtypes = [C.c_float, C.c_float, C.c_float, C.c_int, C.c_int, C.c_void_p, C.c_int]
@@ -165,6 +185,7 @@ def ref_frame_features_in_area(x, y, r, min_level=-1, max_level=-1):
     return out[:n].copy()
 
 
+@_rec.entry("ref_frame_is_in_frustum_points", ref_frame_available, ref_only=True)
 def ref_frame_is_in_frustum_points(Tcw, K, bounds, log_scale_factor, n_levels, cos_limit, pos, normal, min_dist, max_dist):
     """Frame::isInFrustum(MapPoint*) of the reference itself -> (inview, proj, level, viewcos, Ow as the frame derives it)."""
     n = len(pos)
@@ -175,6 +196,7 @@ def ref_frame_is_in_frustum_points(Tcw, K, bounds, log_scale_factor, n_levels, c
     return inview, proj, level, vc, Ow
 
 
+@_rec.entry("ref_frame_is_in_frustum_lines", ref_frame_available, ref_only=True)
 def ref_frame_is_in_frustum_lines(Tcw, K, bounds, log_scale_factor, cos_limit, pos, normal, min_dist, max_dist):
     n = len(pos)
     T = _f32(Tcw); Kc = _f32(K); b = _f32(bounds); mn = _f32(min_dist); mx = _f32(max_dist)
@@ -242,7 +264,10 @@ class RefOrb:
 
     def __init__(self, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20, min_th=7, ordered_heap=True):
         self.nlevels, self.nfeatures, self.ordered_heap = nlevels, nfeatures, ordered_heap
-        self.h = ref_lib().ref_orb_create(nfeatures, scale_factor, nlevels, ini_th, min_th)
+        self.live = ref_orb_available()
+        self.args = (nfeatures, scale_factor, nlevels, ini_th, min_th, ordered_heap)
+        self.last = None       # the last extracted image: level() returns its pyramid
+        self.h = ref_lib().ref_orb_create(nfeatures, scale_factor, nlevels, ini_th, min_th) if self.live else None
 
     def __del__(self):
         if getattr(self, "h", None):
@@ -250,12 +275,22 @@ class RefOrb:
             self.h = None
 
     def tables(self):
+        return _rec.call("RefOrb.tables", self.args, self.live, self._tables)
+
+    def extract(self, img):
+        self.last = _rec.digest("RefOrb.image", img)
+        return _rec.call("RefOrb.extract", (self.args, img), self.live, lambda: self._extract(img))
+
+    def level(self, l):
+        return _rec.call("RefOrb.level", (self.args, self.last, l), self.live, lambda: self._level(l))
+
+    def _tables(self):
         n = self.nlevels
         sc, isc, s2, is2 = (np.zeros(n, np.float32) for _ in range(4))
         ref_lib().ref_orb_tables(self.h, _p(sc), _p(isc), _p(s2), _p(is2))
         return dict(scale=sc, inv_scale=isc, sigma2=s2, inv_sigma2=is2)
 
-    def extract(self, img):
+    def _extract(self, img):
         img = np.ascontiguousarray(img, np.uint8)
         cap = self.nfeatures * 2 + 64
         kps = np.zeros(cap, KP_DTYPE)
@@ -265,7 +300,7 @@ class RefOrb:
         assert 0 <= n <= cap, n
         return kps[:n].copy(), desc[:n].copy()
 
-    def level(self, l):
+    def _level(self, l):
         w, h = C.c_int(), C.c_int()
         ref_lib().ref_orb_level(self.h, l, None, C.byref(w), C.byref(h))
         out = np.zeros((h.value, w.value), np.uint8)
@@ -381,6 +416,7 @@ KL_DTYPE = np.dtype([("startX", "<f4"), ("startY", "<f4"), ("endX", "<f4"), ("en
                      ("lineLength", "<f4"), ("angle", "<f4"), ("octave", "<i4")])
 
 
+@_rec.entry("descriptor_distance", ref_match_available)
 def descriptor_distance(a, b, impl="oracle"):
     a = np.ascontiguousarray(a, np.uint8); b = np.ascontiguousarray(b, np.uint8)
     f = _fn("descriptor_distance", impl); f.argtypes = [C.c_void_p, C.c_void_p]
@@ -394,6 +430,7 @@ def assign_grid(keys, bounds):
     return start, items[:n]
 
 
+@_rec.entry("search_for_initialization", ref_match_available)
 def search_for_initialization(k1, d1, k2, d2, bounds, prev_matched, window=100, nnratio=0.9, check_ori=True, impl="oracle"):
     k1 = np.ascontiguousarray(k1); k2 = np.ascontiguousarray(k2)
     d1 = np.ascontiguousarray(d1, np.uint8); d2 = np.ascontiguousarray(d2, np.uint8)
@@ -406,6 +443,7 @@ def search_for_initialization(k1, d1, k2, d2, bounds, prev_matched, window=100, 
     return nm, m[:len(k1)], pm
 
 
+@_rec.entry("search_by_projection_last", ref_match_available)
 def search_by_projection_last(kc, dc, bounds, Tcw, K, scale_factors, last_valid, last_pos, last_desc, last_octave,
                               last_angle, th, check_ori=True, preassigned=None, impl="oracle"):
     kc = np.ascontiguousarray(kc); dc = np.ascontiguousarray(dc, np.uint8)
@@ -424,6 +462,7 @@ def search_by_projection_last(kc, dc, bounds, Tcw, K, scale_factors, last_valid,
     return nm, m[:len(kc)]
 
 
+@_rec.entry("search_by_projection_points", ref_match_available)
 def search_by_projection_points(k, d, bounds, scale_factors, in_view, proj, level, view_cos, mp_desc, th, nnratio=0.8,
                                 preassigned=None, impl="oracle"):
     k = np.ascontiguousarray(k); d = np.ascontiguousarray(d, np.uint8)
@@ -447,6 +486,7 @@ def bf_knn2(d1, d2):
     return idx[:len(d1)], dist[:len(d1)]
 
 
+@_rec.entry("frame_bf_match", ref_match_available)
 def frame_bf_match(d1, d2, th=50.0, nnratio=0.7, impl="oracle"):
     d1 = np.ascontiguousarray(d1, np.uint8); d2 = np.ascontiguousarray(d2, np.uint8)
     m = np.zeros(max(len(d1), 1), np.int32)
@@ -456,6 +496,7 @@ def frame_bf_match(d1, d2, th=50.0, nnratio=0.7, impl="oracle"):
     return m[:len(d1)]
 
 
+@_rec.entry("search_double", ref_match_available)
 def search_double(d1, d2, nnratio=0.7, impl="oracle"):
     d1 = np.ascontiguousarray(d1, np.uint8); d2 = np.ascontiguousarray(d2, np.uint8)
     m = np.zeros(max(len(d1), 1), np.int32)
@@ -602,6 +643,7 @@ def assign_grid_lines(kl68, bounds):
     return start, items[:n]
 
 
+@_rec.entry("line_search_by_projection_last", ref_match_available)
 def line_search_by_projection_last(kl68, lfunc, desc, bounds, last_valid, proj, last_desc, last_length, th, preassigned=None, impl="oracle"):
     k = _compact_kl(kl68); m = np.zeros(max(len(k), 1), np.int32)
     f = _fn("line_search_by_projection_last", impl)
@@ -614,6 +656,7 @@ def line_search_by_projection_last(kl68, lfunc, desc, bounds, last_valid, proj, 
     return nm, m[:len(k)]
 
 
+@_rec.entry("line_search_by_projection_lines", ref_match_available)
 def line_search_by_projection_lines(kl68, lfunc, desc, bounds, in_view, proj, view_cos, ml_desc, th, nnratio=0.7, preassigned=None, impl="oracle"):
     k = _compact_kl(kl68); m = np.zeros(max(len(k), 1), np.int32)
     f = _fn("line_search_by_projection_lines", impl)
@@ -708,6 +751,7 @@ def _csr(fv):
     return nodes, start, np.array(items, np.int32).reshape(-1)
 
 
+@_rec.entry("search_for_triangulation", ref_match_available)
 def search_for_triangulation(k1, d1, has_mp1, k2, d2, has_mp2, fv1, fv2, F12, Cw1, R2w, t2w, K2, scale_factors2, level_sigma2_2,
                              check_orientation=True, impl="oracle"):
     k1 = np.ascontiguousarray(k1, KP_DTYPE); k2 = np.ascontiguousarray(k2, KP_DTYPE)
@@ -723,6 +767,7 @@ def search_for_triangulation(k1, d1, has_mp1, k2, d2, has_mp2, fv1, fv2, F12, Cw
     return nm, out
 
 
+@_rec.entry("fuse_search", ref_match_available)
 def fuse_search(keys, desc, bounds, Tcw, Ow, K, scale_factors, inv_level_sigma2, log_scale_factor, skip, pos, normal, min_dist,
                 max_dist, mp_desc, th=3.0, impl="oracle"):
     keys = np.ascontiguousarray(keys, KP_DTYPE); desc = np.ascontiguousarray(desc, np.uint8)
@@ -740,6 +785,7 @@ def fuse_search(keys, desc, bounds, Tcw, Ow, K, scale_factors, inv_level_sigma2,
     return bi, f(*args)
 
 
+@_rec.entry("lsd_search_for_triangulation", ref_match_available)
 def lsd_search_for_triangulation(d1, has_ml1, d2, has_ml2, nnratio=0.8, is_double=True, th=80.0, impl="oracle"):
     """LSDmatcher::SearchForTriangulation(pKF1, pKF2, vMatchedPairs, isDouble) (LSDmatcher.cpp:727-776)."""
     d1 = np.ascontiguousarray(d1, np.uint8).reshape(-1, 32); d2 = np.ascontiguousarray(d2, np.uint8).reshape(-1, 32)
@@ -750,6 +796,7 @@ def lsd_search_for_triangulation(d1, has_ml1, d2, has_ml2, nnratio=0.8, is_doubl
     return nm, out
 
 
+@_rec.entry("search_by_bow", ref_match_available)
 def search_by_bow(kK, dK, has_mp_kf, kF, dF, fvK, fvF, nnratio=0.7, check_orientation=True, impl="oracle"):
     """ORBmatcher::SearchByBoW(pKF, F, vpMapPointMatches) (ORBmatcher.cc:187-327) -> (nmatches, matchesF[nF])."""
     kK = np.ascontiguousarray(kK, KP_DTYPE); kF = np.ascontiguousarray(kF, KP_DTYPE)
@@ -763,6 +810,7 @@ def search_by_bow(kK, dK, has_mp_kf, kF, dF, fvK, fvF, nnratio=0.7, check_orient
     return nm, out
 
 
+@_rec.entry("search_by_projection_keyframe", ref_match_available)
 def search_by_projection_keyframe(kc, dc, bounds, Tcw, Ow, K, scale_factors, log_scale_factor, kf_valid, pos, mp_desc, min_dist,
                                   max_dist, kf_angle, th, orb_dist, check_orientation=True, preassigned=None, impl="oracle"):
     """ORBmatcher::SearchByProjection(CurrentFrame, pKF, sAlreadyFound, th, ORBdist) (ORBmatcher.cc:1587-1716).
@@ -787,6 +835,7 @@ def search_by_projection_keyframe(kc, dc, bounds, Tcw, Ow, K, scale_factors, log
     return nm, out
 
 
+@_rec.entry("search_by_bow_keyframes", ref_match_available)
 def search_by_bow_keyframes(k1, d1, mp1, k2, d2, mp2, fv1, fv2, nnratio=0.75, check_orientation=True, impl="oracle"):
     """ORBmatcher::SearchByBoW(pKF1, pKF2, vpMatches12) (ORBmatcher.cc:574-709) -> (nmatches, matches12[n1])."""
     k1 = np.ascontiguousarray(k1, KP_DTYPE); k2 = np.ascontiguousarray(k2, KP_DTYPE)
@@ -809,6 +858,7 @@ def distinctive_descriptors(desc, offsets):
     return best
 
 
+@_rec.entry("ref_distinctive_descriptors", ref_match_available, ref_only=True)
 def ref_distinctive_descriptors(desc, offsets):
     """MapPoint::ComputeDistinctiveDescriptors of the reference itself -> the 32 bytes each point ends up with."""
     desc = np.ascontiguousarray(desc, np.uint8).reshape(-1, 32); off = np.ascontiguousarray(offsets, np.int32)
@@ -818,6 +868,7 @@ def ref_distinctive_descriptors(desc, offsets):
     return out
 
 
+@_rec.entry("predict_scale", ref_match_available)
 def predict_scale(dist, max_dist, log_scale_factor, n_levels, impl="oracle"):
     """MapPoint::PredictScale(currentDist, pKF): the oracle's restatement, or (impl="ref") the reference itself."""
     d = _f32(dist); mx = _f32(max_dist); out = np.zeros(len(d), np.int32)
@@ -830,6 +881,7 @@ def ref_predict_scale(dist, max_dist, log_scale_factor, n_levels):
     return predict_scale(dist, max_dist, log_scale_factor, n_levels, impl="ref")
 
 
+@_rec.entry("lsd_fuse_search", ref_match_available)
 def lsd_fuse_search(keylines, kf_point_desc, bounds, Tcw, Ow, K, scale_line, log_scale_factor_line, skip, pos, normal, min_dist, max_dist,
                     ml_desc, th=3.0, impl="oracle"):
     """Search half of LSDmatcher::Fuse (LSDmatcher.cpp:860-1011) -> (best_idx, best_dist, stop_at);

@@ -271,7 +271,6 @@ def test_tracking_stage_matches_oracle():
     assert retried >= 2 and t0["n_pt"].max() > 100 and t0["n_line"].max() > 20
 
 
-@pytest.mark.skipif(not oracle.ref_frame_available(), reason="oracle/_ref/libref_frame.so did not travel")
 @pytest.mark.parametrize("K,D,w,h,seed", [(synth.TUM1_K, synth.TUM1_DIST, 640, 480, 16), (synth.EUROC_K, synth.EUROC_DIST, 752, 480, 17)])
 def test_frontend_equals_the_reference_frame_constructor(K, D, w, h, seed):
     """The CUDA front-end against the REFERENCE's own monocular Frame constructor (src/Frame.cc compiled with its ORBextractor,

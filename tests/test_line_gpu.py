@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 import oracle
+from oracle import recorded
 import plslam_b200 as pl
 from plslam_b200 import synth
 
@@ -67,16 +68,19 @@ def test_extract_matches_reference_output(name):
     assert len(kl2) == n_all + 1 and kl2[:-1].tobytes() == want.tobytes(), "all KeyLines of the frame vs the reference's"
 
 
-@pytest.mark.skipif(not oracle.ref_line_available(), reason="oracle/_ref/libref_line.so did not travel")
 def test_extract_matches_live_reference_library():
     # the prebuilt reference library itself on the GPU box's CPU (fresh seeds, not in the fixtures): the CUDA KeyLines through the
     # reference's LBD, and the reference's KeyLines against the CUDA ones
     for w, h, seed in [(640, 480, 31), (752, 480, 32)]:
         img = synth.synth_frame(w, h, seed)
         kl, desc, lf = pl.LINEextractor(1, 1.2, 200, 0.0, width=w, height=h)(img)
-        rk = oracle.ref_lsd_keylines(img)
-        order = np.argsort(-rk["response"], kind="stable")
-        want = rk[order][:201].copy(); want["class_id"] = np.arange(201)
+
+        def top_keylines():
+            rk = oracle.ref_lsd_keylines(img)
+            order = np.argsort(-rk["response"], kind="stable")
+            want = rk[order][:201].copy(); want["class_id"] = np.arange(201)
+            return want
+        want = recorded.call("ref_top_keylines", (img, 200), oracle.ref_line_available(), top_keylines)
         assert kl.tobytes() == want.tobytes(), (w, h, seed)
         assert np.array_equal(desc, oracle.ref_lbd_compute(img, want)), (w, h, seed)
 

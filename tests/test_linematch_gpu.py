@@ -58,7 +58,6 @@ def test_search_by_projection_lines(lines, th):
     assert onm > 20 and nm == onm and np.array_equal(m, om)
 
 
-@pytest.mark.skipif(not oracle.ref_match_available(), reason="oracle/_ref/libref_match.so did not travel")
 def test_line_matchers_equal_the_reference_matcher_code(lines):
     """The CUDA line matchers against the REFERENCE's own LSDmatcher.cpp (compiled into oracle/_ref/libref_match.so, run on this box's
     CPU): SearchDouble and the two projection searches, same inputs, identical match lists."""

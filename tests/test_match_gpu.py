@@ -128,7 +128,6 @@ def test_bf_knn_and_line_matching():
         assert nm == onm and np.array_equal(m, om)
 
 
-@pytest.mark.skipif(not oracle.ref_match_available(), reason="oracle/_ref/libref_match.so did not travel")
 def test_matchers_equal_the_reference_matcher_code(frames):
     """The CUDA matchers against the REFERENCE's own ORBmatcher.cc (compiled into oracle/_ref/libref_match.so, run on this box's CPU):
     SearchForInitialization and the two tracking searches, same inputs, identical match lists."""

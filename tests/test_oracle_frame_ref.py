@@ -11,11 +11,20 @@ import ctypes as C
 import numpy as np
 import pytest
 import oracle
+from oracle import recorded
 from oracle.binding import lib, _p
 from plslam_b200 import synth
 
-pytestmark = pytest.mark.skipif(not oracle.ref_frame_available(), reason="oracle/_ref/libref_frame.so not built (needs /root/reference)")
 NODIST = (0.0, 0.0, 0.0, 0.0, 0.0)
+
+
+def _ref_in_view(name, f, *args):
+    """isInFrustum of the reference -> (inview, then proj / level / viewcos of the points in view only, Ow)"""
+    def run():
+        r = f(*args)
+        inv = r[0].astype(bool)
+        return r[0], r[1][inv], r[2][inv], r[3][inv], r[4]
+    return recorded.call(name, args, oracle.ref_frame_available(), run)
 
 
 def _oracle_frame(img, K, D, nfeatures=1000, nlines=200, mask=None, mll=0.0):
@@ -56,7 +65,9 @@ def test_frame_constructor_with_mask():
 def test_get_features_in_area():
     img = synth.synth_frame(640, 480, 3)
     F = oracle.ref_frame_construct(img, synth.TUM1_K, synth.TUM1_DIST)
-    keysUn, b = F["keysUn"], F["bounds"]
+    O = _oracle_frame(img, synth.TUM1_K, synth.TUM1_DIST)
+    assert O["keysUn"].tobytes() == F["keysUn"].tobytes() and O["bounds"].tobytes() == F["bounds"].tobytes()
+    keysUn, b = O["keysUn"], O["bounds"]        # the frame's own keypoints and bounds (identical bytes)
     rng = np.random.default_rng(0)
     f = lib().oracle_features_in_area
     f.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_int, C.c_int, C.c_void_p]
@@ -75,11 +86,12 @@ def test_is_in_frustum_points(seed, cosl):
     v = synth.synth_map_view(seed, 6000)
     b = oracle.image_bounds(synth.TUM1_K, synth.TUM1_DIST, 640, 480)
     log_sf = float(np.float32(np.log(np.float32(1.2))))
-    ref = oracle.ref_frame_is_in_frustum_points(v["Tcw"], synth.TUM1_K, b, log_sf, 8, cosl, v["pos"], v["normal"], v["min_dist"], v["max_dist"])
+    ref = _ref_in_view("ref_in_view_points", oracle.ref_frame_is_in_frustum_points, v["Tcw"], synth.TUM1_K, b, log_sf, 8, cosl, v["pos"], v["normal"],
+                       v["min_dist"], v["max_dist"])
     got = oracle.is_in_frustum_points(v["Tcw"], ref[4], synth.TUM1_K, b, log_sf, 8, cosl, v["pos"], v["normal"], v["min_dist"], v["max_dist"])
     assert got[0].sum() > 100 and np.array_equal(got[0], ref[0])
     inv = got[0].astype(bool)
-    assert got[1][inv].tobytes() == ref[1][inv].tobytes() and np.array_equal(got[2][inv], ref[2][inv]) and got[3][inv].tobytes() == ref[3][inv].tobytes()
+    assert got[1][inv].tobytes() == ref[1].tobytes() and np.array_equal(got[2][inv], ref[2]) and got[3][inv].tobytes() == ref[3].tobytes()
     # the camera centre the frame derives is the fp32 gemm of -Rcw^T tcw; the synthetic Ow agrees to an ulp or so
     assert np.allclose(ref[4], v["Ow"], rtol=0, atol=1e-5)
 
@@ -91,8 +103,9 @@ def test_is_in_frustum_lines(seed, cosl):
         v["min_dist"] = (v["max_dist"] / 1.2 ** 12).astype(np.float32)
     b = oracle.image_bounds(synth.TUM1_K, synth.TUM1_DIST, 640, 480)
     log_sf = float(np.float32(np.log(np.float32(1.2))))
-    ref = oracle.ref_frame_is_in_frustum_lines(v["Tcw"], synth.TUM1_K, b, log_sf, cosl, v["pos"], v["normal"], v["min_dist"], v["max_dist"])
+    ref = _ref_in_view("ref_in_view_lines", oracle.ref_frame_is_in_frustum_lines, v["Tcw"], synth.TUM1_K, b, log_sf, cosl, v["pos"], v["normal"],
+                       v["min_dist"], v["max_dist"])
     got = oracle.is_in_frustum_lines(v["Tcw"], ref[4], synth.TUM1_K, b, log_sf, cosl, v["pos"], v["normal"], v["min_dist"], v["max_dist"])
     assert got[0].sum() > 50 and np.array_equal(got[0], ref[0])
     inv = got[0].astype(bool)
-    assert got[1][inv].tobytes() == ref[1][inv].tobytes() and np.array_equal(got[2][inv], ref[2][inv]) and got[3][inv].tobytes() == ref[3][inv].tobytes()
+    assert got[1][inv].tobytes() == ref[1].tobytes() and np.array_equal(got[2][inv], ref[2]) and got[3][inv].tobytes() == ref[3].tobytes()

@@ -3,7 +3,7 @@
 oracle/_ref/libref_line.so - oracle/Makefile target `ref`, oracle/ref_line_wrap.cpp, oracle/shim/).
 
 (a) committed reference outputs (tests/golden/line_ref_*.npz, tools/gen_golden_line_ref.py): run everywhere;
-(b) live comparison where libref_line.so exists: every KeyLine record of a frame byte-identical (all 17 fields, including the
+(b) comparison against libref_line.so (live where it is built, elsewhere its recorded outputs, oracle/recorded.py): every KeyLine record of a frame byte-identical (all 17 fields, including the
     libm-dependent angle), 32-byte LBD descriptors AND the 72-float LBD vectors bit-identical.
 """
 import os
@@ -11,13 +11,13 @@ import sys
 import numpy as np
 import pytest
 import oracle
+from oracle import recorded
 from plslam_b200 import synth
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
 from gen_golden_line_ref import CASES, select  # noqa: E402
 
 G = os.path.join(os.path.dirname(__file__), "golden")
-needs_ref = pytest.mark.skipif(not oracle.ref_line_available(), reason="oracle/_ref/libref_line.so not built (needs /root/reference)")
 
 
 def _oracle_all_keylines(img, mask=None):
@@ -25,6 +25,14 @@ def _oracle_all_keylines(img, mask=None):
     KeyLine that `resize(index + 1)` appends when nothing is cut, LineExtractor.cpp:64)"""
     kl, desc, lf = oracle.line_extract(img, mask=mask, nfeatures=100000)
     return kl[:-1]
+
+
+def _ref_all_keylines(img, mask=None):
+    """every KeyLine the reference's detector makes for the frame, put in LINEextractor's sorted order by select()"""
+    def run():
+        rk = oracle.ref_lsd_keylines(img, mask)
+        return select(rk, len(rk))
+    return recorded.call("ref_all_keylines", (img, mask), oracle.ref_line_available(), run)
 
 
 @pytest.mark.parametrize("name", sorted(CASES))
@@ -45,26 +53,23 @@ def test_oracle_equals_committed_reference_output(name):
     assert np.array_equal(d2, g["desc"]) and dv.tobytes() == g["desvec"].tobytes()
 
 
-@needs_ref
 @pytest.mark.parametrize("w,h,seed", [(640, 480, 3), (640, 480, 7), (752, 480, 9), (1241, 376, 10), (320, 240, 3), (800, 600, 12)])
 def test_keylines_equal_live_reference(w, h, seed):
     img = synth.synth_frame(w, h, seed)
-    rk = oracle.ref_lsd_keylines(img)
+    rk = _ref_all_keylines(img)
     assert len(rk) > 100
-    assert _oracle_all_keylines(img).tobytes() == select(rk, len(rk)).tobytes()
+    assert _oracle_all_keylines(img).tobytes() == rk.tobytes()
 
 
-@needs_ref
 def test_keylines_with_mask_equal_live_reference():
     img = synth.synth_frame(640, 480, 4)
     mask = np.full((480, 640), 255, np.uint8)
     mask[100:300, 150:500] = 0          # a line is dropped only if BOTH end points fall on zeros (LSDDetector_custom.cpp:203-213)
-    rk = oracle.ref_lsd_keylines(img, mask)
-    assert len(rk) < len(oracle.ref_lsd_keylines(img))
-    assert _oracle_all_keylines(img, mask).tobytes() == select(rk, len(rk)).tobytes()
+    rk = _ref_all_keylines(img, mask)
+    assert len(rk) < len(_ref_all_keylines(img))
+    assert _oracle_all_keylines(img, mask).tobytes() == rk.tobytes()
 
 
-@needs_ref
 @pytest.mark.parametrize("w,h,seed,nf", [(640, 480, 3, 200), (752, 480, 9, 200), (1241, 376, 10, 400), (320, 240, 3, 100)])
 def test_lbd_equals_live_reference(w, h, seed, nf):
     img = synth.synth_frame(w, h, seed)
@@ -76,20 +81,22 @@ def test_lbd_equals_live_reference(w, h, seed, nf):
     assert ov.tobytes() == rv.tobytes()                     # the 72 floats behind the bits as well
 
 
-@needs_ref
 def test_lbd_on_short_and_border_lines():
     # lines clipped at the border and very short lines exercise the coordinate clamps and the 2-pixel support region
     img = synth.synth_frame(640, 480, 8)
-    rk = oracle.ref_lsd_keylines(img)
-    sel = rk[(rk["lineLength"] < 6) | (rk["startPointX"] < 3) | (rk["endPointY"] > 475) | (rk["startPointY"] < 3) | (rk["endPointX"] > 635)][:150].copy()
+
+    def short_and_border_lines():
+        rk = oracle.ref_lsd_keylines(img)
+        sel = rk[(rk["lineLength"] < 6) | (rk["startPointX"] < 3) | (rk["endPointY"] > 475) | (rk["startPointY"] < 3) | (rk["endPointX"] > 635)][:150].copy()
+        sel["class_id"] = np.arange(len(sel))
+        return sel
+    sel = recorded.call("ref_short_and_border_lines", (img,), oracle.ref_line_available(), short_and_border_lines, full=True)
     assert len(sel) > 20
-    sel["class_id"] = np.arange(len(sel))
     rd, rv = oracle.ref_lbd_compute(img, sel, want_float=True)
     od, ov = oracle.lbd_compute(img, sel, want_float=True)
     assert np.array_equal(od, rd) and ov.tobytes() == rv.tobytes()
 
 
-@needs_ref
 @pytest.mark.parametrize("w,h,seed,nf,mll", [(640, 480, 1, 200, 0.0), (640, 480, 2, 200, 0.0), (752, 480, 5, 300, 0.0), (1241, 376, 4, 200, 0.0),
                                              (640, 480, 3, 150, 20.0), (640, 480, 6, 400, 30.0), (320, 240, 3, 100, 0.0)])
 def test_line_extractor_equals_live_reference(w, h, seed, nf, mll):
@@ -97,22 +104,27 @@ def test_line_extractor_equals_live_reference(w, h, seed, nf, mll):
     the min_line_length cut, class ids, line equations through Eigen's cross product) over its own detector and descriptor."""
     img = synth.synth_frame(w, h, seed)
     ok, od, ol = oracle.line_extract(img, nfeatures=nf, min_line_length=mll)
-    rk, rd, rl = oracle.ref_line_extract(img, nfeatures=nf, min_line_length=mll)
-    assert len(ok) == len(rk) > 50
-    if ok.tobytes() != rk.tobytes():
+
+    def split():
+        # the reference's output with the rows that differ from the oracle's (`bad`) apart from the rest
+        rk, rd, rl = oracle.ref_line_extract(img, nfeatures=nf, min_line_length=mll)
+        bad = np.array([i for i in range(min(len(ok), len(rk))) if ok[i].tobytes() != rk[i].tobytes()], np.int64)
+        keep = np.setdiff1d(np.arange(len(rk)), bad)
+        return len(rk), bad, rk[bad], rk[keep], rd[keep], rl[keep]
+    n_ref, bad, rk_bad, rk, rd, rl = recorded.call("ref_line_extract_split", (img, nf, mll, ok), oracle.ref_line_available(), split)
+    assert len(ok) == n_ref > 50
+    if len(bad):
         # LineExtractor.cpp:43 sorts with std::sort, which is not stable: lines with EQUAL response (equal length) may come out in
         # either order (the oracle and the CUDA path keep detection order).  Anything else must match; undo such swaps and compare.
-        bad = [i for i in range(len(ok)) if ok[i].tobytes() != rk[i].tobytes()]
-        assert all(ok["response"][i] == rk["response"][i] for i in bad) and len(bad) <= 4, bad
-        key = lambda k: [tuple(r) for r in np.sort(k[bad][["startPointX", "startPointY", "endPointX", "endPointY"]].copy(), order=["startPointX", "startPointY"])]
-        assert key(ok) == key(rk)
-        keep = np.setdiff1d(np.arange(len(ok)), bad)
-        ok, od, ol, rk, rd, rl = ok[keep], od[keep], ol[keep], rk[keep], rd[keep], rl[keep]
+        assert all(ok["response"][i] == rk_bad["response"][j] for j, i in enumerate(bad)) and len(bad) <= 4, bad
+        key = lambda rows: [tuple(r) for r in np.sort(rows[["startPointX", "startPointY", "endPointX", "endPointY"]].copy(), order=["startPointX", "startPointY"])]
+        assert key(ok[bad]) == key(rk_bad)
+    keep = np.setdiff1d(np.arange(len(ok)), bad)
+    ok, od, ol = ok[keep], od[keep], ol[keep]
     assert ok.tobytes() == rk.tobytes() and np.array_equal(od, rd)
     assert ol.tobytes() == rl.tobytes()          # the three fp64 coefficients of every line equation, bit for bit
 
 
-@needs_ref
 def test_line_extractor_with_mask_equals_live_reference():
     img = synth.synth_frame(640, 480, 4)
     mask = np.zeros((480, 640), np.uint8); mask[14:465, 14:625] = 255        # the geometry of masks/mask.png

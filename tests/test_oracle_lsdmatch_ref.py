@@ -12,7 +12,6 @@ from plslam_b200 import synth
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from test_localmap2 import _line_fuse_problem, _args  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not oracle.ref_match_available(), reason="oracle/_ref/libref_match.so not built (needs /root/reference)")
 BOUNDS = [0.0, 0.0, 640.0, 480.0]
 
 

@@ -65,7 +65,6 @@ def test_extract_matches_reference_output(name):
     assert [tuple(d) for d in g["level_dims"]] == [ex.mvImagePyramid(l).shape[::-1] for l in range(nl)]
 
 
-@pytest.mark.skipif(not oracle.ref_orb_available(), reason="oracle/_ref/libref_orb.so did not travel")
 def test_extract_matches_live_reference_library():
     # the prebuilt reference library itself, run on the GPU box's CPU next to the CUDA path (fresh seeds, not in the fixtures)
     for w, h, seed, nf in [(640, 480, 21, 1000), (752, 480, 22, 1000), (1241, 376, 23, 2000)]:

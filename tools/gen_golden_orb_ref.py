@@ -14,7 +14,6 @@ import plslam_b200  # noqa  (synth only; no GPU needed)
 from plslam_b200 import synth
 import oracle
 
-assert oracle.ref_orb_available(), "needs /root/reference (make -C oracle ref)"
 out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
 
@@ -37,6 +36,7 @@ CASES = {"640x480_n1000": ("synth", 640, 480, 1, 1000, 1.2, 8), "640x480_n2000":
          "640x480_sparse": ("sparse", 640, 480, 0, 1000, 1.2, 8), "640x480_n500_s11": ("synth", 640, 480, 11, 500, 1.2, 8)}
 
 if __name__ == "__main__":
+    assert oracle.ref_orb_available(), "needs oracle/_ref/libref_orb.so (make -C oracle ref, where the reference tree exists)"
     for name, (kind, w, h, seed, nf, sf, nl) in CASES.items():
         im = frame(kind, w, h, seed)
         r = oracle.RefOrb(nf, sf, nl, 20, 7)
